@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- fwd+bwd throughput of the Gaussian feature rasterizer on BASELINE.json's headline config.
 
-    python bench.py --gpus N --steps K --warmup W [--impl ours|reference]
+    python bench.py --gpus N --steps K --warmup W [--impl ours|reference] [--dump-outputs DIR]
 
 * workload (config.workload): BASELINE.json configs[1] = synthetic 1M Gaussians, 1080x1920, K=32, one
   camera per GPU per step (SYN(P,H,W,K,cam) of BASELINE.md section 2.2; camera index = rank).
@@ -19,14 +19,23 @@
              taken by the library on its launch stream in a SEPARATE pass of the same steps (the instrumentation costs
              ~18 event records per step, so it stays out of the `value` region); algorithmic bytes per launch as in DESIGN.md.
 * `c4`     : BASELINE.json configs[3] (3M Gaussians, 8 cameras, STRONG scaling: 8 / N cameras per rank, one all-reduce of
-             the 384 MB feature gradient per 8-camera batch), measured in the same run after the headline numbers.
+             the 384 MB feature gradient per 8-camera batch), measured in the same run after the headline numbers, over
+             --steps batches like the headline; --no-c4 skips it (with --impl reference, whose batches are far slower, this leg
+             dominates the run time at the default --steps).
 * `cpu_baseline`: the CPU oracle port (oracle/sagars_oracle.c, OpenMP over tiles) timed on the host cores on the
              same workload (rank 0, N=1 only).
-* `--impl reference`: the UNMODIFIED reference extension (oracle/_ref, rebuilt for sm_100a from /root/reference by
+* `--impl reference`: the UNMODIFIED reference extension (oracle/_ref, rebuilt for sm_100a from the reference's sources by
              oracle/build_ref.py) through its own GaussianRasterizer API on the same inputs.  NOTE: the reference has
              no CPU implementation of this path -- its implementation IS the CUDA extension, and the north star's
              ">= 3x the reference CUDA rasterizer" is a ratio against exactly this arm.  If oracle/_ref is absent the
              arm falls back to the CPU oracle port and says so.
+* `--dump-outputs DIR`: after the timed steps, what the last step of the `value` region computed on rank 0 -- the image and
+             radii the forward returned for rank 0's last camera and the gradients of the six inputs it differentiates -- as
+             DIR/<name>.npy (float32).  The gradients are those the step leaves on the leaves: summed over all of rank 0's
+             cameras and, with N > 1, dL_dcolors all-reduced over the ranks; compare dumps of runs with the same workload and
+             the same number of GPUs only.  An array of more than DUMP_MAX_ELEMENTS elements is stored as a fixed, seeded
+             sample of that many elements (the same positions in every run), so two builds can be compared output for output:
+             the inputs are seeded as well.
 """
 import argparse
 import json
@@ -56,12 +65,15 @@ WORKLOADS = {
     # small variant for quick local checks (never a bench line)
     "tiny": dict(P=20_000, H=270, W=480, K=32, cameras=None, desc="tiny smoke workload"),
 }
+DUMP_MAX_ELEMENTS = 1 << 20       # 8 arrays of at most 4 MB each
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200,
+                    help="timed steps of each measured region (value, e2e) and timed batches of the c4 leg (8 cameras each); "
+                         "the per-stage profiling pass runs min(steps, 20)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c2", choices=list(WORKLOADS))
@@ -75,6 +87,8 @@ def parse():
     ap.add_argument("--allreduce", default="nccl", choices=["nccl", "multimem"],
                     help="N > 1, developer switch: 'multimem' = the library's own all-reduce over the NVSwitch multicast mapping")
     ap.add_argument("--binning", default="default", choices=["default", "radix", "tile_sort", "depth_first"], help="developer A/B switch (rasterizer.set_binning)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32; large arrays as a fixed, seeded sample)")
     return ap.parse_args()
 
 
@@ -199,6 +213,7 @@ class Runner:
             if a.allreduce_mode == "overlap":
                 self.reducer = FeatureGradReducer(side_stream=True, reduce_fn=self.own_allreduce.all_reduce_ if self.own_allreduce else None)
         self.last = {}
+        self.keep_color = False                                      # outputs() needs the last step's image
 
     def _settings(self, c, view, proj, campos, bg):
         wl = self.wl
@@ -228,6 +243,8 @@ class Runner:
         for rast in self.rasts:
             color, radii = self._render(rast)
             self.last["grad_fn"], self.last["radii"] = color.grad_fn, radii
+            if self.keep_color:
+                self.last["color"] = color.detach()
             color.backward(self.dL)
         if self.use_dist:
             self._reduce()
@@ -283,6 +300,21 @@ class Runner:
             import torch.distributed as dist
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item())
+
+    def outputs(self):
+        """The last resident step's outputs as float32 host arrays, large ones sampled: image and radii of this rank's last
+        camera; the leaves' gradients, i.e. summed over this rank's cameras and, under torchrun, with dL_dcolors all-reduced."""
+        named = {"color": self.last["color"], "radii": self.last["radii"], "dL_dmeans3D": self.means3D.grad,
+                 "dL_dmeans2D": self.means2D.grad, "dL_dopacities": self.opac.grad, "dL_dscales": self.scales.grad,
+                 "dL_drotations": self.rots.grad, "dL_dcolors": self.colors.grad}
+        out = {}
+        for name, t in named.items():
+            flat = t.detach().reshape(-1)
+            if flat.numel() > DUMP_MAX_ELEMENTS:
+                idx = np.sort(np.random.default_rng(0).choice(flat.numel(), DUMP_MAX_ELEMENTS, replace=False))
+                flat = flat[torch.from_numpy(idx).to(flat.device)]
+            out[name] = flat.float().cpu().numpy()
+        return out
 
     def counters(self, ours: bool):
         """Work counters of this rank's last camera (SURVEY.md section 8(d)), decoded from the last call's scratch."""
@@ -357,10 +389,13 @@ def main():
             Settings, Rast = mod.GaussianRasterizationSettings, mod.GaussianRasterizer
             ref_kind = "reference-cuda-ext"
         else:
+            if a.dump_outputs is not None:
+                raise SystemExit("--dump-outputs needs a CUDA implementation; the CPU fallback of --impl reference has no timed steps")
             from seganygaussians_b200 import synthetic
             return reference_cpu_arm(a, wl, synthetic.scene(P, H, W, K))
 
     run = Runner(a, wl, world, rank, dev, use_dist, Settings, Rast, R)
+    run.keep_color = a.dump_outputs is not None
 
     # ---------------- warm-up, then the timed regions ----------------
     sampler = ClockSampler(local_rank) if rank == 0 else None
@@ -373,6 +408,7 @@ def main():
         _lib.reset_launch_count()
     ms_total = run.timed(run.step_resident, a.steps, sampler)
     launches = _lib.launch_count() if a.impl == "ours" else None
+    dumped = run.outputs() if a.dump_outputs is not None and rank == 0 else None    # before the e2e pass replaces the gradients
     ms_e2e = run.timed(run.step_e2e, a.steps)
     clocks = sampler.result() if sampler else None
     stage, stage_steps = None, min(a.steps, 20)
@@ -400,6 +436,10 @@ def main():
         if use_dist:
             dist.destroy_process_group()
         return 0
+    if dumped is not None:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, arr in dumped.items():
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), arr)
 
     T_tiles = ((W + 15) // 16) * ((H + 15) // 16)
     strong = wl["cameras"] is not None
@@ -487,7 +527,7 @@ def c4_leg(a, world, rank, dev, use_dist, Settings, Rast, R):
     batch is fixed, `value` = 8 * P * H * W * steps / time (max over ranks)."""
     wl = WORKLOADS["c4"]
     n_used = world if use_dist else 1
-    steps = 10 if a.impl == "ours" else 3          # 8 cameras x 3M Gaussians per batch: a reference batch takes ~1 s on one GPU
+    steps = a.steps
     try:
         run = Runner(a, wl, world, rank, dev, use_dist, Settings, Rast, R)
         for _ in range(2):

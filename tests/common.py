@@ -254,6 +254,117 @@ def float_err(a, b):
     return float(np.max(d / tol)), float(np.max(d)), scale
 
 
+# ----------------------------------------------------------------------------------------------
+# sampled golden vectors: outputs of the unmodified reference too large to store whole
+# ----------------------------------------------------------------------------------------------
+GOLDEN_SAMPLES = 128
+GOLDEN_BLOCKS = 32
+
+
+def _block_sums(flat: np.ndarray, nblocks: int) -> np.ndarray:
+    """(sum a, sum |a|) over each of ``nblocks`` contiguous, near-equal blocks of a flat array, in float64: shape (2, nblocks)."""
+    f = np.asarray(flat, np.float64)
+    edges = (np.arange(nblocks, dtype=np.int64) * f.size) // nblocks
+    return np.stack([np.add.reduceat(f, edges), np.add.reduceat(np.abs(f), edges)])
+
+
+def digest(a) -> np.ndarray:
+    """SHA-256 of an array's shape, dtype and bytes, as 32 uint8: stands in for the array where equality must be exact."""
+    import hashlib
+    a = np.ascontiguousarray(np.asarray(a))
+    h = hashlib.sha256(repr((a.shape, a.dtype.str)).encode())
+    h.update(a.tobytes())
+    return np.frombuffer(h.digest(), np.uint8)
+
+
+def summarize(name: str, a, exact: bool = False, samples: int = GOLDEN_SAMPLES, seed: int = 0) -> dict:
+    """The entries a sampled golden file keeps of one array: its digest when it must match exactly; otherwise a seeded
+    sample of elements (most of them where the array is non-zero), ``meta`` = (max |a|, sum |a|, *shape) and ``blocks`` =
+    sum a and sum |a| over GOLDEN_BLOCKS contiguous blocks of the flat array (for a per-Gaussian array: ranges of Gaussians;
+    for an image: bands of rows).  max |a| is the tolerance's absolute scale (float_err), so a sampled comparison applies the
+    same bound as one over the whole array."""
+    a = np.asarray(a)
+    if exact:
+        return {name + ".digest": digest(a)}
+    flat = a.reshape(-1).astype(np.float32)
+    rng = np.random.default_rng(seed)
+    nz = np.flatnonzero(flat)
+    parts = [rng.choice(flat.size, min(samples // 4, flat.size), replace=False)]
+    if nz.size:
+        parts.append(rng.choice(nz, min(samples - parts[0].size, nz.size), replace=False))
+    idx = np.unique(np.concatenate(parts)).astype(np.int32)
+    meta = [np.abs(flat).max() if flat.size else 0.0, np.abs(flat.astype(np.float64)).sum()] + list(a.shape)
+    return {name + ".idx": idx, name + ".val": flat[idx], name + ".meta": np.array(meta, np.float64),
+            name + ".blocks": _block_sums(flat, min(GOLDEN_BLOCKS, flat.size)).astype(np.float32)}
+
+
+def check_summary(z, name: str, a, rtol: float = RTOL, atol_scale: float = ATOL_SCALE):
+    """Compare an array with its entries in a sampled golden file ``z``.  Returns (ok, report line).
+
+    Sampled elements must meet the elementwise bound of float_err (scale = max |ref| of the whole array).  max |a|, sum |a|
+    and, per block, sum a and sum |a| are checked against the bounds that the elementwise one implies for them
+    (|sum a - sum b| <= sum |a - b| <= rtol * (sum |a| + sum |b|) + atol_scale * scale * n), so an error confined to a part of
+    the array (a range of Gaussians, a band of rows) that is large enough to move its block's sums is caught even where no
+    sample lies.  The block sums are stored in float32: their rounding (1e-6 of the block's sum |ref|) is allowed for."""
+    if name + ".digest" in z:
+        ok = np.array_equal(digest(a), z[name + ".digest"])
+        return ok, f"  EXACT {name:22s} " + ("equal" if ok else "DIFFERS")
+    a = np.asarray(a)
+    meta = z[name + ".meta"]
+    scale, ref_sum, shape = float(meta[0]), float(meta[1]), tuple(int(s) for s in meta[2:])
+    if a.shape != shape:
+        return False, f"  FLOAT {name:22s} shape {a.shape} vs {shape}  MISMATCH"
+    flat = np.asarray(a, np.float64).reshape(-1)
+    x, v = flat[z[name + ".idx"]], np.asarray(z[name + ".val"], np.float64)
+    r = d = 0.0
+    if x.size:
+        diff = np.abs(x - v)
+        r = float(np.max(diff / (rtol * np.maximum(np.abs(x), np.abs(v)) + atol_scale * scale + 1e-30)))
+        d = float(diff.max())
+    amax, asum = float(np.abs(flat).max()) if flat.size else 0.0, float(np.abs(flat).sum())
+    max_ok = abs(amax - scale) <= rtol * max(amax, scale) + atol_scale * scale + 1e-30
+    sum_ok = abs(asum - ref_sum) <= rtol * (asum + ref_sum) + atol_scale * scale * flat.size + 1e-30
+    ref_blocks = np.asarray(z[name + ".blocks"], np.float64)
+    nb = ref_blocks.shape[1]
+    blocks = _block_sums(flat, nb)
+    n_b = np.diff(np.append((np.arange(nb, dtype=np.int64) * flat.size) // nb, flat.size))
+    block_tol = rtol * (blocks[1] + ref_blocks[1]) + atol_scale * scale * n_b + 1e-6 * ref_blocks[1] + 1e-30
+    block_r = float(np.max(np.abs(blocks - ref_blocks) / block_tol)) if nb else 0.0
+    ok = r <= 1.0 and max_ok and sum_ok and block_r <= 1.0 and not bool(np.isnan(flat).any())
+    return ok, (f"  FLOAT {name:22s} samples={z[name + '.idx'].size} max|d|={d:.3e} tol-ratio={r:.3f} max|a|={amax:.6e}/{scale:.6e} "
+                f"sum|a|={asum:.6e}/{ref_sum:.6e} block-tol-ratio={block_r:.3f}" + ("" if ok else "  MISMATCH"))
+
+
+# what a sampled golden file keeps of a runner output (run_torch_impl): integer state and final_T exactly, the rest sampled
+SUMMARY_EXACT = INT_FWD + ("final_T",)
+SUMMARY_FLOAT = ("color", "out_mask", "out_depth") + GRADS + ("means2D", "conic_opacity", "depths", "cov3D")
+
+
+def summary_arrays(o) -> dict:
+    """``{name: array}`` of a runner output for compare_summaries (fields the runner left as None are absent)."""
+    return {f: getattr(o, f) for f in SUMMARY_EXACT + SUMMARY_FLOAT if getattr(o, f, None) is not None}
+
+
+def summarize_all(arrays: dict, exact=()) -> dict:
+    out = {}
+    for name, a in arrays.items():
+        out.update(summarize(name, a, exact=name in exact))
+    return out
+
+
+def compare_summaries(z, arrays: dict, skip=()):
+    """check_summary over ``{name: array}``; every name in the file but those in ``skip`` must be given.
+    Returns (ok, report lines)."""
+    stored = {f.rsplit(".", 1)[0] for f in z.files if f != "config"} - set(skip)
+    lines = [f"  names: stored {sorted(stored)} given {sorted(arrays)}"] if stored != set(arrays) else []
+    ok = not lines
+    for name in sorted(set(arrays) & stored):
+        o, line = check_summary(z, name, arrays[name])
+        ok &= o
+        lines.append(line)
+    return ok, lines
+
+
 def compare(a, b, ints=INT_FWD, floats=FLOAT_FWD + GRADS, verbose=True):
     """Compare two runner outputs. Returns (ok, report lines)."""
     ok = True

@@ -19,3 +19,11 @@ def clouds():
     out["flat_1500"] = flat
     out["tiny_5"] = rng.random((5, 3), dtype=np.float32)
     return out
+
+
+def scene_cloud():
+    """300k points shaped like a scene's initial point cloud, with floaters far away from the bulk."""
+    rng = np.random.default_rng(2)
+    big = (rng.standard_normal((300000, 3)) * np.array([5, 1, 3])).astype(np.float32)
+    big[:1000] *= 40
+    return big

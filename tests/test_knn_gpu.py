@@ -1,7 +1,6 @@
 """GPU: sagars_knn (csrc/knn.cu) through its Python wrapper and the two import stand-ins (SURVEY.md section 8(f) rank 1)
-against the brute-force oracle, and -- when oracle/_ref/simple_knn is present -- against the unmodified reference
-extension (fp32 rounding level: rtol 1e-6)."""
-import importlib.util
+against the brute-force oracle, and against golden outputs of the unmodified reference extension (fp32 rounding level:
+rtol 1e-6)."""
 import os
 import sys
 
@@ -10,20 +9,10 @@ import pytest
 import torch
 
 from oracle import knn_oracle
-from tests import knn_cases
+from tests import common, knn_cases
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-def _ref_distcuda2():
-    so = os.path.join(ROOT, "oracle", "_ref", "simple_knn", "_C.so")
-    if not os.path.exists(so):
-        return None
-    spec = importlib.util.spec_from_file_location("_C", so)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod.distCUDA2
 
 
 @pytest.mark.parametrize("name", list(knn_cases.clouds()))
@@ -61,23 +50,21 @@ def test_separate_query_set():
 
 
 def test_distcuda2_shim_matches_live_reference():
-    ref = _ref_distcuda2()
-    if ref is None:
-        pytest.skip("oracle/_ref/simple_knn not built")
+    """distCUDA2 against the reference's simple_knn._C.distCUDA2 on a B200: its whole output on the small clouds, a sampled
+    golden vector (plus max and sum of the whole output) on a 300k-point scene cloud."""
     sys.path.append(os.path.join(ROOT, "seganygaussians_b200", "shims"))
     from simple_knn._C import distCUDA2
-    cases = dict(knn_cases.clouds())
-    rng = np.random.default_rng(2)
-    big = (rng.standard_normal((300000, 3)) * np.array([5, 1, 3])).astype(np.float32)
-    big[:1000] *= 40                                               # floaters far away from the bulk
-    cases["scene_300k"] = big
-    for name, pts in cases.items():
+    golden = os.path.join(ROOT, "tests", "golden", "knn")
+    small = np.load(os.path.join(golden, "simple_knn_small.npz"))
+    for name, pts in knn_cases.clouds().items():
         if len(pts) < 4:
             continue
-        t = torch.from_numpy(pts).cuda()
-        ours, theirs = distCUDA2(t).cpu().numpy(), ref(t).float().cpu().numpy()
+        ours, theirs = distCUDA2(torch.from_numpy(pts).cuda()).cpu().numpy(), small[name]
         # both are exact 3-NN searches in fp32; the mean differs by a few ulps at most (FMA contraction of the distances)
         assert np.allclose(ours, theirs, rtol=1e-6, atol=0), (name, float((np.abs(ours - theirs) / theirs).max()))
+    ours = distCUDA2(torch.from_numpy(knn_cases.scene_cloud()).cuda()).cpu().numpy()
+    ok, line = common.check_summary(np.load(os.path.join(golden, "simple_knn_scene_300k.npz")), "scene_300k", ours, rtol=1e-6, atol_scale=0)
+    assert ok, line
 
 
 def test_knn_points_shim():

@@ -1,7 +1,8 @@
 """GPU parity tests (run with `-m gpu` on a B200): the CUDA path, driven through the reference-shaped operator
 API (which calls the C ABI), against (1) the CPU oracle on seeded inputs, (2) golden vectors of the unmodified
-reference, (3) the unmodified reference extension itself when oracle/_ref is present, and (4) size-independent
-properties at BASELINE.json's full size.  Integer state is compared exactly; fp32 within RTOL=1e-4 (tests/common.py)."""
+reference, (3) sampled golden vectors of the unmodified reference extension up to BASELINE.json's full sizes
+(tests/golden/reference, tests/golden/make_golden_sampled.py), and (4) size-independent properties at BASELINE.json's
+full size.  Integer state is compared exactly; fp32 within RTOL=1e-4 (tests/common.py)."""
 import glob
 import os
 
@@ -15,6 +16,7 @@ from seganygaussians_b200 import synthetic
 pytestmark = pytest.mark.gpu
 
 GOLDEN = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "*.npz")))
+REF_GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "reference")
 
 
 @pytest.fixture(scope="module", autouse=True)
@@ -73,21 +75,19 @@ LIVE_REF = [("cf_medium", 200000, 540, 960, 32, False), ("base_medium", 100000, 
 
 @pytest.mark.parametrize("cfg", LIVE_REF, ids=[c[0] for c in LIVE_REF])
 def test_cuda_matches_live_reference(cfg):
-    """Against the unmodified reference extension on the same GPU, up to BASELINE.json's full size (c2)."""
-    _, P, H, W, K, depth = cfg
-    if not common.have_ref(common.variant_of(K, depth)):
-        pytest.skip("oracle/_ref not built (python oracle/build_ref.py where /root/reference is mounted)")
+    """Against the outputs of the unmodified reference extension on a B200, up to BASELINE.json's full size (c2): integer state
+    and final_T to the bit, images, gradients and per-Gaussian state within the parity tolerance (sampled golden vectors)."""
+    name, P, H, W, K, depth = cfg
+    z = np.load(os.path.join(REF_GOLDEN, name + ".npz"))
     sc = synthetic.scene(P, H, W, K)
-    ref = common.run_torch_impl("ref", sc, K, depth=depth)
     for tensor_cores in (True, False):
         ours = common.run_torch_impl("ours", sc, K, depth=depth, tensor_cores=tensor_cores)
-        ok, lines = common.compare(ours, ref, floats=common.FLOAT_FWD + common.GRADS + ("means2D", "conic_opacity", "depths", "cov3D"),
-                                   verbose=False)
-        assert ok, f"tensor_cores={tensor_cores}\n" + "\n".join(lines)
-        assert np.array_equal(ours.final_T, ref.final_T)
+        arrays = common.summary_arrays(ours)
         if not tensor_cores:
             # fp32 SIMT path: images are not merely close, the per-pixel arithmetic is kept operation for operation
-            assert np.array_equal(ours.color, ref.color)
+            arrays["color_bits"] = ours.color
+        ok, lines = common.compare_summaries(z, arrays, skip=("color_bits",) if tensor_cores else ())
+        assert ok, f"tensor_cores={tensor_cores}\n" + "\n".join(lines)
 
 
 # BASELINE.json configs[2] / [3] / [4] at their full sizes, default kernels only (the small LIVE_REF cases above also run the fp32 SIMT
@@ -99,19 +99,15 @@ LIVE_REF_LARGE = [("c3_like_5M", 5_000_000, 1036, 1600, 32, False, False), ("c4_
 
 @pytest.mark.parametrize("cfg", LIVE_REF_LARGE, ids=[c[0] for c in LIVE_REF_LARGE])
 def test_cuda_matches_live_reference_at_baseline_sizes(cfg):
-    """Integer state exact, final_T bit-equal, images and all gradients within 1e-4 of the unmodified reference extension."""
-    _, P, H, W, K, depth, use_sh = cfg
-    if not common.have_ref(common.variant_of(K, depth)):
-        pytest.skip("oracle/_ref not built (python oracle/build_ref.py where /root/reference is mounted)")
+    """Integer state exact, final_T bit-equal, images and all gradients within 1e-4 of the unmodified reference extension
+    (sampled golden vectors of its outputs on a B200)."""
+    name, P, H, W, K, depth, use_sh = cfg
+    z = np.load(os.path.join(REF_GOLDEN, name + ".npz"))
     sc = synthetic.scene(P, H, W, K, sh_coeffs=16 if use_sh else 0)
-    kw = dict(depth=depth, use_sh=use_sh, sh_degree=3 if use_sh else 0)
-    ref = common.run_torch_impl("ref", sc, K, **kw)
-    torch.cuda.empty_cache()
-    ours = common.run_torch_impl("ours", sc, K, **kw)
-    ok, lines = common.compare(ours, ref, floats=common.FLOAT_FWD + common.GRADS + ("means2D", "conic_opacity", "depths", "cov3D"), verbose=False)
+    ours = common.run_torch_impl("ours", sc, K, depth=depth, use_sh=use_sh, sh_degree=3 if use_sh else 0)
+    ok, lines = common.compare_summaries(z, common.summary_arrays(ours))
     assert ok, "\n".join(lines)
-    assert np.array_equal(ours.final_T, ref.final_T)
-    assert ours.num_rendered == ref.num_rendered and ours.num_rendered > 2 * P // 3
+    assert ours.num_rendered > 2 * P // 3
 
 
 def _render(sc, K, colors=None, bg=None, opac=None, cov_precomp=None, use_cub=False, debug=False, backward=False, dL=None,
@@ -215,17 +211,23 @@ def test_cov3d_precomp_path_matches_scale_rotation_path():
     assert float((a - b).abs().max()) < 5e-3 and float((a - b).abs().mean()) < 1e-5
 
 
-def test_mark_visible_matches_the_oracle_and_the_reference():
-    """a2 / a18: `markVisible` point by point -- a cloud that straddles the camera's near plane (view z > 0.2), against the CPU
-    oracle (oracle/sagars_oracle.c, `in_frustum`) and against the unmodified reference's own `GaussianRasterizer.markVisible`."""
-    from seganygaussians_b200 import rasterizer as R
-    from oracle import oracle as orc
-    dev = torch.device("cuda", 0)
+def mark_visible_cloud():
+    """(points, camera): a cloud that straddles the camera's near plane (view z > 0.2)."""
     sc = synthetic.scene(64, 40, 56, 32)
     c = sc.cam
     g = torch.Generator().manual_seed(11)
     pts = c.camera_center[None] + (torch.rand(20000, 3, generator=g) - 0.5) * 8.0          # all around the camera
-    pts = torch.cat([pts, sc.gauss.means3D, (c.camera_center[None] * 3.0).repeat(7, 1)]).contiguous()
+    return torch.cat([pts, sc.gauss.means3D, (c.camera_center[None] * 3.0).repeat(7, 1)]).contiguous(), c
+
+
+def test_mark_visible_matches_the_oracle_and_the_reference():
+    """a2 / a18: `markVisible` point by point on a cloud that straddles the camera's near plane, against the CPU oracle
+    (oracle/sagars_oracle.c, `in_frustum`) and against the unmodified reference's own `GaussianRasterizer.markVisible`
+    (its result on a B200, stored as a digest)."""
+    from seganygaussians_b200 import rasterizer as R
+    from oracle import oracle as orc
+    dev = torch.device("cuda", 0)
+    pts, c = mark_visible_cloud()
     rs = R.GaussianRasterizationSettings(40, 56, c.tanfovx, c.tanfovy, torch.zeros(32, device=dev), 1.0, c.world_view_transform.to(dev),
                                          c.full_proj_transform.to(dev), 0, c.camera_center.to(dev), False, False)
     ours = R.GaussianRasterizerContrastiveF(rs).markVisible(pts.to(dev))
@@ -233,13 +235,8 @@ def test_mark_visible_matches_the_oracle_and_the_reference():
     want = orc.mark_visible(pts.numpy(), c.world_view_transform.numpy())
     assert 0.2 < want.mean() < 0.8                                                           # the cloud really straddles the plane
     assert np.array_equal(ours.cpu().numpy(), want)
-    if common.have_ref("cf"):
-        ref = common.ref_module("cf")
-        rs_ref = ref.GaussianRasterizationSettings(40, 56, c.tanfovx, c.tanfovy, torch.zeros(32, device=dev), 1.0,
-                                                   c.world_view_transform.to(dev), c.full_proj_transform.to(dev), 0,
-                                                   c.camera_center.to(dev), False, False)
-        theirs = ref.GaussianRasterizer(rs_ref).markVisible(pts.to(dev))
-        assert torch.equal(ours, theirs.to(torch.bool))
+    ok, line = common.check_summary(np.load(os.path.join(REF_GOLDEN, "mark_visible.npz")), "visible", ours.cpu().numpy())
+    assert ok, line
 
 
 def test_edge_cases():

@@ -1,14 +1,14 @@
 """SURVEY.md section 8 rows a19 / a20: the drop-in ``gaussian_renderer`` against the REFERENCE's own ``gaussian_renderer``.
 
 Both bindings are driven with the same duck-typed camera / model / pipe objects (SURVEY.md Appendix F): the reference's
-``render``, ``render_mask``, ``render_with_depth`` and ``render_contrastive_feature`` run on top of the reference's own CUDA
-extensions (``oracle/_ref``, installed by ``oracle/build_ref.py``), ours on top of libsagars; result dictionaries and the
-gradients that flow back into the model's leaves are compared (integer outputs exact, fp32 within the parity tolerance).
-Also the DEPTH variant's mask-only API (``GaussianRasterizer.forward_mask``) against the reference's own ``forward_mask``."""
-import importlib
+``render``, ``render_mask``, ``render_with_depth`` and ``render_contrastive_feature``, run on a B200 on top of the reference's
+own CUDA extensions, left sampled golden vectors of their result dictionaries and of the gradients that flow back into the
+model's leaves (tests/golden/reference, tests/golden/make_golden_sampled.py); ours run on top of libsagars and are compared
+with them (integer outputs exact, fp32 within the parity tolerance).  Also the DEPTH variant's mask-only API
+(``GaussianRasterizer.forward_mask``) against the reference's own ``forward_mask``."""
 import importlib.util
+import math
 import os
-import sys
 from types import SimpleNamespace
 
 import numpy as np
@@ -20,47 +20,17 @@ from seganygaussians_b200 import synthetic
 
 pytestmark = pytest.mark.gpu
 ROOT = common.ROOT
-REF_RENDERER = os.path.join(common.REF_DIR, "renderer")
+REF_GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "reference")
+EXACT_OUTPUTS = ("out.radii", "out.visibility_filter", "out.viewspace_points")
 
 
-@pytest.fixture(autouse=True)
-def _restore_import_state():
-    """The reference's python packages are put in front of sys.path for these tests only: afterwards the path entry and the
-    modules imported from it are removed again (other tests import the DROP-IN ``gaussian_renderer`` by that same name)."""
-    saved_path = list(sys.path)
-    yield
-    sys.path[:] = saved_path
-    for k in [k for k in list(sys.modules) if k.split(".")[0] in ("gaussian_renderer", "scene", "utils", "arguments")]:
-        f = getattr(sys.modules[k], "__file__", None) or ""
-        if os.path.realpath(f).startswith(os.path.realpath(common.REF_DIR)) or not f:
-            del sys.modules[k]
-
-
-def _load_bindings():
-    """(reference gaussian_renderer bound to the reference extensions, our drop-in bound to libsagars)."""
-    if not (os.path.exists(os.path.join(REF_RENDERER, "gaussian_renderer", "__init__.py")) and
-            all(common.have_ref(v) for v in ("base", "cf", "depth"))):
-        pytest.skip("oracle/_ref (extensions + renderer binding) not built: python oracle/build_ref.py where /root/reference is mounted")
-    import seganygaussians_b200 as S
-    if S.SHIMS_DIR not in sys.path:
-        sys.path.append(S.SHIMS_DIR)                      # plyfile / pytorch3d stand-ins for the reference's `scene` package
-    for p in (REF_RENDERER, common.REF_DIR):              # the reference's python packages and its extensions win
-        if p in sys.path:
-            sys.path.remove(p)
-        sys.path.insert(0, p)
-    for name in ("gaussian_renderer", "scene", "utils", "arguments"):
-        mod = sys.modules.get(name)
-        if mod is not None and not os.path.realpath(getattr(mod, "__file__", None) or "/").startswith(os.path.realpath(common.REF_DIR)):
-            for k in [k for k in sys.modules if k == name or k.startswith(name + ".")]:
-                del sys.modules[k]
-    ref = importlib.import_module("gaussian_renderer")
-    assert os.path.realpath(ref.__file__).startswith(os.path.realpath(REF_RENDERER)), ref.__file__
-    assert os.path.realpath(sys.modules["diff_gaussian_rasterization"].__file__).startswith(os.path.realpath(common.REF_DIR))
+def _load_ours():
+    """Our drop-in ``gaussian_renderer`` (bound to libsagars), under a name of its own."""
     spec = importlib.util.spec_from_file_location("sagars_gaussian_renderer",
                                                   os.path.join(ROOT, "seganygaussians_b200", "dropin", "gaussian_renderer", "__init__.py"))
     ours = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(ours)
-    return ref, ours
+    return ours
 
 
 class _Model:
@@ -86,10 +56,15 @@ class _Model:
     get_point_features = property(lambda s: s._point_features)
 
     def get_covariance(self, scaling_modifier=1):
-        # the reference's build_covariance_from_scaling_rotation (scene/gaussian_model.py:33-37): L = R S, Sigma = L L^T, 6 unique
-        from utils.general_utils import build_scaling_rotation, strip_symmetric
-        L = build_scaling_rotation(scaling_modifier * self._scaling, self._rotation)
-        return strip_symmetric(L @ L.transpose(1, 2))
+        # what the reference's build_covariance_from_scaling_rotation computes (scene/gaussian_model.py:33-37): R from the
+        # normalised quaternion, L = R S, Sigma = L L^T, the 6 unique entries
+        r, x, y, z = torch.nn.functional.normalize(self._rotation, dim=1).unbind(1)
+        R = torch.stack([1 - 2 * (y * y + z * z), 2 * (x * y - r * z), 2 * (x * z + r * y),
+                         2 * (x * y + r * z), 1 - 2 * (x * x + z * z), 2 * (y * z - r * x),
+                         2 * (x * z - r * y), 2 * (y * z + r * x), 1 - 2 * (x * x + y * y)], dim=1).view(-1, 3, 3)
+        L = R * (scaling_modifier * self._scaling)[:, None, :]
+        S = L @ L.transpose(1, 2)
+        return S[:, [0, 0, 0, 1, 1, 2], [0, 1, 2, 1, 2, 2]]
 
     def leaves(self):
         return {"xyz": self._xyz, "opacity": self._opacity, "scaling": self._scaling, "rotation": self._rotation, "sh": self._sh,
@@ -102,15 +77,9 @@ class _Model:
 
 def _camera(sc, dev):
     c = sc.cam
-    import math
     return SimpleNamespace(FoVx=2 * math.atan(c.tanfovx), FoVy=2 * math.atan(c.tanfovy), image_height=sc.H, image_width=sc.W,
                            feature_height=sc.H, feature_width=sc.W, world_view_transform=c.world_view_transform.to(dev),
                            full_proj_transform=c.full_proj_transform.to(dev), camera_center=c.camera_center.to(dev))
-
-
-def _close(got, want, what):
-    r, d, s = common.float_err(got.detach().cpu().numpy(), want.detach().cpu().numpy())
-    assert r <= 1.0, f"{what}: max|d|={d:.3e} max|ref|={s:.3e} tol-ratio={r:.2f}"
 
 
 def _run(fn, model, loss_keys, dL, **kw):
@@ -132,10 +101,13 @@ CASES = [("render", dict(), ("render",)),
          ("render_contrastive_feature", dict(call_kw=dict(norm_point_features=True)), ("render",))]
 
 
-@pytest.mark.parametrize("case", CASES, ids=[f"{c[0]}-{i}" for i, c in enumerate(CASES)])
-def test_dropin_render_functions_match_the_reference_binding(case):
+def golden_name(i, case):
+    return f"dropin_{i}_{case[0]}"
+
+
+def case_inputs(case):
+    """(function name, keyword arguments, loss keys, upstream gradients, model) of one case: seeded, so identical every run."""
     name, opt, loss_keys = case
-    ref, ours = _load_bindings()
     dev = torch.device("cuda", 0)
     P, H, W, K = 30000, 200, 304, 32
     sc = synthetic.scene(P, H, W, K)
@@ -152,47 +124,52 @@ def test_dropin_render_functions_match_the_reference_binding(case):
         kw["filtered_mask"] = (torch.arange(P, device=dev) % 7) == 0
     gen = torch.Generator().manual_seed(11)
     dL = {"render": (torch.randn(nch, H, W, generator=gen) / (H * W)).to(dev), "mask": (torch.randn(1 if name == "render_with_depth" else 3, H, W, generator=gen) / (H * W)).to(dev)}
-    o_ref, g_ref = _run(getattr(ref, name), model, loss_keys, dL, **kw)
+    return name, kw, loss_keys, dL, model
+
+
+def result_arrays(out, grads):
+    """``{name: array}`` of a render call's result dictionary and of the gradients of the model's leaves (None: absent)."""
+    arrays = {"out." + k: v.detach().cpu().numpy() for k, v in out.items()}
+    arrays.update({"grad." + n: g.cpu().numpy() for n, g in grads.items() if g is not None})
+    return arrays
+
+
+@pytest.mark.parametrize("case", CASES, ids=[f"{c[0]}-{i}" for i, c in enumerate(CASES)])
+def test_dropin_render_functions_match_the_reference_binding(case):
+    ours = _load_ours()
+    z = np.load(os.path.join(REF_GOLDEN, golden_name(CASES.index(case), case) + ".npz"))
+    name, kw, loss_keys, dL, model = case_inputs(case)
     o_our, g_our = _run(getattr(ours, name), model, loss_keys, dL, **kw)
-    assert set(o_ref) == set(o_our)
-    assert torch.equal(o_ref["radii"], o_our["radii"]) and torch.equal(o_ref["visibility_filter"], o_our["visibility_filter"])
-    for k in o_ref:
-        if k not in ("radii", "visibility_filter", "viewspace_points"):
-            assert o_ref[k].shape == o_our[k].shape, k
-            _close(o_our[k], o_ref[k], f"{name}[{k}]")
-    for n in g_ref:
-        assert (g_ref[n] is None) == (g_our[n] is None), n
-        if g_ref[n] is not None:
-            _close(g_our[n], g_ref[n], f"{name}: d/d{n}")
-    assert g_ref["viewspace_points"].abs().max() > 0
+    ok, lines = common.compare_summaries(z, result_arrays(o_our, g_our))
+    assert ok, "\n".join(lines)
+    assert g_our["viewspace_points"].abs().max() > 0
 
 
-def test_forward_mask_matches_the_reference_forward_mask():
-    """DEPTH ``GaussianRasterizer.forward_mask`` (reference diff_gaussian_rasterization_depth/__init__.py:359-391): image and the
-    gradient of the per-Gaussian mask against the reference's own mask-only kernels."""
-    if not common.have_ref("depth"):
-        pytest.skip("oracle/_ref not built")
-    from seganygaussians_b200 import rasterizer as R
-    refmod = common.ref_module("depth")
+def forward_mask_run(Settings, Rast):
+    """(image, radii, dL/dmask) of ``forward_mask`` of a DEPTH rasterizer class on a seeded scene."""
     dev = torch.device("cuda", 0)
     P, H, W = 20000, 160, 240
     sc = synthetic.scene(P, H, W, 3)
     g, c = sc.gauss, sc.cam
     gen = torch.Generator().manual_seed(3)
     dL = (torch.randn(1, H, W, generator=gen) / (H * W)).to(dev)
-    res = {}
-    for tag, Settings, Rast in (("ref", refmod.GaussianRasterizationSettings, refmod.GaussianRasterizer),
-                                ("ours", R.GaussianRasterizationSettings, R.GaussianRasterizerDepth)):
-        rs = Settings(image_height=H, image_width=W, tanfovx=c.tanfovx, tanfovy=c.tanfovy, bg=torch.zeros(3, device=dev), scale_modifier=1.0,
-                      viewmatrix=c.world_view_transform.to(dev), projmatrix=c.full_proj_transform.to(dev), sh_degree=0,
-                      campos=c.camera_center.to(dev), prefiltered=False, debug=False)
-        mask = (torch.rand(P, 1, generator=torch.Generator().manual_seed(7)) * 0.5 + 0.5).to(dev).requires_grad_(True)
-        out = Rast(raster_settings=rs).forward_mask(means3D=g.means3D.to(dev), means2D=torch.zeros(P, 3, device=dev), opacities=g.opacities.to(dev),
-                                                    mask=mask, scales=g.scales.to(dev), rotations=g.rotations.to(dev), cov3D_precomp=None)
-        img, radii = out[0], out[-1]
-        (img * dL).sum().backward()
-        res[tag] = (img.detach(), radii.detach(), mask.grad.detach())
-    assert torch.equal(res["ref"][1], res["ours"][1])
-    _close(res["ours"][0], res["ref"][0], "forward_mask image")
-    _close(res["ours"][2], res["ref"][2], "forward_mask dL/dmask")
-    assert res["ref"][2].abs().max() > 0
+    rs = Settings(image_height=H, image_width=W, tanfovx=c.tanfovx, tanfovy=c.tanfovy, bg=torch.zeros(3, device=dev), scale_modifier=1.0,
+                  viewmatrix=c.world_view_transform.to(dev), projmatrix=c.full_proj_transform.to(dev), sh_degree=0,
+                  campos=c.camera_center.to(dev), prefiltered=False, debug=False)
+    mask = (torch.rand(P, 1, generator=torch.Generator().manual_seed(7)) * 0.5 + 0.5).to(dev).requires_grad_(True)
+    out = Rast(raster_settings=rs).forward_mask(means3D=g.means3D.to(dev), means2D=torch.zeros(P, 3, device=dev), opacities=g.opacities.to(dev),
+                                                mask=mask, scales=g.scales.to(dev), rotations=g.rotations.to(dev), cov3D_precomp=None)
+    img, radii = out[0], out[-1]
+    (img * dL).sum().backward()
+    return img.detach().cpu().numpy(), radii.detach().cpu().numpy(), mask.grad.detach().cpu().numpy()
+
+
+def test_forward_mask_matches_the_reference_forward_mask():
+    """DEPTH ``GaussianRasterizer.forward_mask`` (reference diff_gaussian_rasterization_depth/__init__.py:359-391): image and the
+    gradient of the per-Gaussian mask against the reference's own mask-only kernels (sampled golden vectors)."""
+    from seganygaussians_b200 import rasterizer as R
+    img, radii, dmask = forward_mask_run(R.GaussianRasterizationSettings, R.GaussianRasterizerDepth)
+    z = np.load(os.path.join(REF_GOLDEN, "forward_mask.npz"))
+    ok, lines = common.compare_summaries(z, {"image": img, "radii": radii, "dL_dmask": dmask})
+    assert ok, "\n".join(lines)
+    assert np.abs(dmask).max() > 0
