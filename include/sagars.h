@@ -74,9 +74,7 @@ enum {
 #define SAGARS_FLAG_FWD_WARP_ANY 256u /* forward: the warp-per-block tensor-core kernel for every colour-only channel count
                                         (default: only C = 32; other counts use the fp32 SIMT kernel, bit-exact colours)  */
 
-#define SAGARS_FLAG_STAGE_TMA 512u   /* tile-per-CTA fp32 forward (render_forward.cu): gather the per-instance records / feature rows
-                                        with bulk asynchronous copies (cp.async.bulk, TMA unit) completing on mbarriers instead of
-                                        16-byte cp.async pieces.  Identical results; opt-in until measured (DESIGN.md section 4)   */
+/* 512u: unassigned and ignored.  Callers built against earlier v4 headers may still set it, so it is not reused */
 
 #define SAGARS_FLAG_TILE_SORT 1024u  /* binning without a global sort: per-tile instance counts -> scan -> scatter -> one CTA per tile
                                         sorts its own segment (tile_sort.cu) instead of duplicate + 6 radix passes + range

@@ -29,7 +29,6 @@ FLAG_BWD_TILE = 128
 FLAG_BWD_TC = 2048
 FLAG_DEPTH_FIRST = 4096
 FLAG_FWD_WARP_ANY = 256
-FLAG_STAGE_TMA = 512
 FLAG_TILE_SORT = 1024
 
 ERROR_NAMES = {0: "OK", 1: "EINVAL", 2: "ECUDA", 3: "ENOCOLOR", 4: "EALLOC", 5: "EPREFILTER"}

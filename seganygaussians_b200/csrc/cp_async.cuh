@@ -1,5 +1,5 @@
-// cp_async.cuh -- thin wrappers over the asynchronous global->shared copy instructions used to stage
-// per-tile instance lists (LDGSTS) and, for contiguous runs, bulk copies completed on an mbarrier.
+// cp_async.cuh -- thin wrappers over the asynchronous global->shared copy instructions (LDGSTS) used to stage
+// per-tile instance lists, and over the vectorised global reductions.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -33,37 +33,6 @@ template <int N>
 __device__ __forceinline__ void cp_async_wait_group()
 {
     asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory");
-}
-
-// ---- bulk asynchronous copies (the TMA engine's non-tensor form) completing on an mbarrier ----
-// One instruction moves `bytes` (a multiple of 16; source and destination 16-byte aligned) from global to shared memory;
-// the mbarrier's transaction count drops by `bytes` when the data has landed.  Used to GATHER per-instance rows
-// (32-byte records, K*4-byte feature rows): one bulk copy per row, no per-thread address arithmetic or register staging.
-__device__ __forceinline__ void mbarrier_init(uint64_t* bar, uint32_t arrivals)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(arrivals) : "memory");
-}
-// make the initialised barrier (and earlier generic-proxy writes to shared memory) visible to the async proxy
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void mbarrier_arrive_expect_tx(uint64_t* bar, uint32_t tx_bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(tx_bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_copy_g2s(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(smem_dst)), "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-// Wait for the phase of the given parity.  A wait that does not end within ~2^26 polls (seconds; a copy that can never
-// complete, e.g. a misaligned row) traps: a CUDA error the caller sees instead of a hung GPU.
-__device__ __forceinline__ void mbarrier_wait_parity(uint64_t* bar, uint32_t parity)
-{
-    uint32_t ok = 0;
-    for (uint32_t spins = 0; !ok; spins++) {
-        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                     : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-        if (!ok && spins > (1u << 26)) __trap();
-    }
 }
 
 // vectorised fire-and-forget global reductions (sm_90+): one instruction adds 4 / 2 floats

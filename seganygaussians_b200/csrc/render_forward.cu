@@ -14,11 +14,7 @@
 //     256-instance batch);
 //   * a (warp, splat) pair in which no pixel can pass the reference's tests (power <= 0 and a conservative
 //     per-splat lower bound on power that implies alpha >= 1/255) is rejected with one warp vote, before expf;
-//   * C is a run-time value (<= 64), dispatched onto float4-group templates;
-//   * SAGARS_FLAG_STAGE_TMA selects a second staging engine for the same kernel body: the 32-byte records and
-//     (K % 4 == 0) the K*4-byte feature rows of a batch are gathered by bulk asynchronous copies (cp.async.bulk, the
-//     TMA unit's non-tensor form: ONE instruction per row, issued by warp 0, no per-thread 16-byte pieces) that complete
-//     on an mbarrier per pipeline stage; consumers wait on the barrier's phase instead of cp.async.wait_all.
+//   * C is a run-time value (<= 64), dispatched onto float4-group templates.
 // The per-pixel arithmetic (power, alpha, the 1/255 and 1e-4 tests, the order of accumulation)
 // is kept operation for operation so that n_contrib / final_T / colours match the reference.
 #include "common.cuh"
@@ -28,12 +24,12 @@
 
 namespace sagars {
 
-template <int NQ, bool VEC, bool MD, bool COLOR, bool TMA>
-static int launch_fwd_tt(const sagars_forward_args& a, const Dims& d, GeomView g, ImageView im,
-                         const uint32_t* point_list, const float* features, cudaStream_t s, bool debug)
+template <int NQ, bool VEC, bool MD, bool COLOR>
+static int launch_fwd_t(const sagars_forward_args& a, const Dims& d, GeomView g, ImageView im,
+                        const uint32_t* point_list, const float* features, cudaStream_t s, bool debug)
 {
-    auto kern = TMA ? render_forward_tma_kernel<NQ, VEC, MD, COLOR> : render_forward_kernel<NQ, VEC, MD, COLOR>;
-    const size_t smem = sizeof(typename FwdSmemSel<NQ, TMA>::type);
+    auto kern = render_forward_kernel<NQ, VEC, MD, COLOR>;
+    const size_t smem = sizeof(FwdSmem<NQ>);
     {   // opt in to the dynamic shared-memory size once per device (not on every launch: the call takes the context lock)
         static DeviceOnce once;
         int dev = 0;
@@ -48,14 +44,6 @@ static int launch_fwd_tt(const sagars_forward_args& a, const Dims& d, GeomView g
                                       im.final_T, im.n_contrib, a.out_color, a.out_mask, a.out_depth);
     SAGARS_LAUNCH_CHECK(s, debug);
     return SAGARS_OK;
-}
-
-template <int NQ, bool VEC, bool MD, bool COLOR>
-static int launch_fwd_t(const sagars_forward_args& a, const Dims& d, GeomView g, ImageView im,
-                        const uint32_t* point_list, const float* features, cudaStream_t s, bool debug)
-{
-    if (a.flags & SAGARS_FLAG_STAGE_TMA) return launch_fwd_tt<NQ, VEC, MD, COLOR, true>(a, d, g, im, point_list, features, s, debug);
-    return launch_fwd_tt<NQ, VEC, MD, COLOR, false>(a, d, g, im, point_list, features, s, debug);
 }
 
 int launch_render_forward(const sagars_forward_args& a, const Dims& d, GeomView g, ImageView im,

@@ -1,6 +1,5 @@
 // render_forward_kernels.cuh -- the device code of render_forward.cu (see there).  Free of host-side runtime calls so that
-// tests/test_render_forward_emulated.py can compile these kernels for the CPU against tests/cuda_emu/ (both staging engines:
-// cp.async pieces and bulk copies on mbarriers) and run them against the oracle.
+// tests/test_render_forward_emulated.py can compile the kernel for the CPU against tests/cuda_emu/ and run it against the oracle.
 #pragma once
 #include "common.cuh"
 #include "cp_async.cuh"
@@ -23,60 +22,13 @@ struct FwdSmem {
     float depthv[2][FWD_BATCH];         // DEPTH variant: per-instance view depth
 };
 
-template <int NQ>
-struct FwdSmemTma : FwdSmem<NQ> {
-    uint64_t bar[2];                    // one mbarrier per pipeline stage (bulk-copy staging only)
-};
-template <int NQ, bool TMA>
-struct FwdSmemSel { using type = FwdSmem<NQ>; };
-template <int NQ>
-struct FwdSmemSel<NQ, true> { using type = FwdSmemTma<NQ>; };
-
-// bulk-copy staging of one batch: warp 0 announces the bytes of the batch on the stage's mbarrier and gathers the
-// rows, one cp.async.bulk per row (record: 32 B; feature row: K*4 B when K % 4 == 0)
-template <int NQ, bool VEC, bool COLOR>
-__device__ __forceinline__ void fwd_issue_batch_bulk(FwdSmemTma<NQ>& sm, int stage, int idbuf, int cnt, int K,
-                                                     const float* __restrict__ geo, const float* __restrict__ features)
-{
-    if (threadIdx.x >= 32) return;
-    const int lane = threadIdx.x;
-    const uint32_t row_bytes = (VEC && COLOR) ? (uint32_t)K * 4u : 0u;
-    uint64_t* bar = &sm.bar[stage];
-    if (lane == 0) mbarrier_arrive_expect_tx(bar, (uint32_t)cnt * (32u + row_bytes));
-    __syncwarp();
-    for (int j = lane; j < cnt; j += 32) {
-        const uint32_t id = sm.ids[idbuf][j];
-        bulk_copy_g2s(&sm.geo[stage][j][0], geo + 8 * (size_t)id, 32u, bar);
-        if (VEC && COLOR) bulk_copy_g2s(&sm.feat[stage][j][0], features + (size_t)id * K, row_bytes, bar);
-    }
-}
-
 // issue the asynchronous copies of one batch (ids already in smem)
-template <int NQ, bool VEC, bool MD, bool COLOR, bool TMA = false>
-__device__ __forceinline__ void fwd_issue_batch(typename FwdSmemSel<NQ, TMA>::type& sm, int stage, int idbuf, int cnt, int K,
+template <int NQ, bool VEC, bool MD, bool COLOR>
+__device__ __forceinline__ void fwd_issue_batch(FwdSmem<NQ>& sm, int stage, int idbuf, int cnt, int K,
                                                 const float* __restrict__ geo, const float* __restrict__ features,
                                                 const float* __restrict__ mask, const float* __restrict__ depths)
 {
     const int tid = threadIdx.x;
-    if constexpr (TMA) {
-        fwd_issue_batch_bulk<NQ, VEC, COLOR>(sm, stage, idbuf, cnt, K, geo, features);
-        if (MD) {
-            if (tid < cnt) {
-                const uint32_t id = sm.ids[idbuf][tid];
-                sm.maskv[stage][tid] = mask[id];
-                sm.depthv[stage][tid] = depths[id];
-            }
-        }
-        if (COLOR && !VEC) {
-            float* f = reinterpret_cast<float*>(&sm.feat[stage][0][0]);
-            for (int c = tid; c < cnt * K; c += TILE_PIX) {
-                const int j = c / K, k = c - j * K;
-                const uint32_t id = sm.ids[idbuf][j];
-                f[j * (4 * NQ) + k] = features[(size_t)id * K + k];
-            }
-        }
-        return;
-    }
     // geometry records: 2 x 16 B per instance
     for (int c = tid; c < cnt * 2; c += TILE_PIX) {
         const int j = c >> 1, h = c & 1;
@@ -119,18 +71,17 @@ __device__ __forceinline__ void fwd_pad_batch(FwdSmem<NQ>& sm, int stage, int cn
     }
 }
 
-template <int NQ, bool VEC, bool MD, bool COLOR, bool TMA>
-__device__ __forceinline__ void
-render_forward_body(const uint2* __restrict__ ranges, const uint32_t* __restrict__ point_list,
-                    int W, int H, int K,
-                    const float* __restrict__ geo, const float* __restrict__ features,
-                    const float* __restrict__ mask, const float* __restrict__ depths, const float* __restrict__ bg,
-                    float* __restrict__ final_T, uint32_t* __restrict__ n_contrib,
-                    float* __restrict__ out_color, float* __restrict__ out_mask, float* __restrict__ out_depth)
+template <int NQ, bool VEC, bool MD, bool COLOR>
+__global__ void __launch_bounds__(TILE_PIX)
+render_forward_kernel(const uint2* __restrict__ ranges, const uint32_t* __restrict__ point_list,
+                      int W, int H, int K,
+                      const float* __restrict__ geo, const float* __restrict__ features,
+                      const float* __restrict__ mask, const float* __restrict__ depths, const float* __restrict__ bg,
+                      float* __restrict__ final_T, uint32_t* __restrict__ n_contrib,
+                      float* __restrict__ out_color, float* __restrict__ out_mask, float* __restrict__ out_depth)
 {
     SAGARS_DYNAMIC_SMEM(smem_raw);
-    using Smem = typename FwdSmemSel<NQ, TMA>::type;
-    Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
+    FwdSmem<NQ>& sm = *reinterpret_cast<FwdSmem<NQ>*>(smem_raw);
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int tiles_x = gridDim.x;
@@ -150,15 +101,6 @@ render_forward_body(const uint2* __restrict__ ranges, const uint32_t* __restrict
         float* f = reinterpret_cast<float*>(&sm.feat[0][0][0]);
         for (int c = tid; c < 2 * FWD_BATCH * 4 * NQ; c += TILE_PIX) f[c] = 0.f;
     }
-    if constexpr (TMA) {
-        if (tid == 0) {
-            mbarrier_init(&sm.bar[0], 1);
-            mbarrier_init(&sm.bar[1], 1);
-        }
-        // the barriers and the zero fill above (generic proxy) before the first bulk copy (async proxy) touches them;
-        // the __syncthreads of the prologue below orders every thread's fence before warp 0 issues
-        fence_proxy_async_smem();
-    }
 
     float T = 1.0f;
     uint32_t last_contributor = 0;
@@ -172,11 +114,10 @@ render_forward_body(const uint2* __restrict__ ranges, const uint32_t* __restrict
     if (nbatch > 0) {
         if (tid < min(FWD_BATCH, total)) sm.ids[0][tid] = point_list[range.x + tid];
         __syncthreads();
-        fwd_issue_batch<NQ, VEC, MD, COLOR, TMA>(sm, 0, 0, min(FWD_BATCH, total), K, geo, features, mask, depths);
-        if constexpr (!TMA) cp_async_commit();
+        fwd_issue_batch<NQ, VEC, MD, COLOR>(sm, 0, 0, min(FWD_BATCH, total), K, geo, features, mask, depths);
+        cp_async_commit();
         if (nbatch > 1 && tid < min(FWD_BATCH, total - FWD_BATCH)) sm.ids[1][tid] = point_list[range.x + FWD_BATCH + tid];
-        if constexpr (TMA) mbarrier_wait_parity(&sm.bar[0], 0u);
-        else cp_async_wait_all();
+        cp_async_wait_all();
         fwd_pad_batch<NQ>(sm, 0, min(FWD_BATCH, total));
         __syncthreads();
     }
@@ -189,9 +130,9 @@ render_forward_body(const uint2* __restrict__ ranges, const uint32_t* __restrict
 
         // (A) start the copies of batch b+1 (its ids were stored one iteration ago)
         if (b + 1 < nbatch) {
-            fwd_issue_batch<NQ, VEC, MD, COLOR, TMA>(sm, stage ^ 1, (b + 1) & 1, min(FWD_BATCH, total - (b + 1) * FWD_BATCH),
-                                              K, geo, features, mask, depths);
-            if constexpr (!TMA) cp_async_commit();
+            fwd_issue_batch<NQ, VEC, MD, COLOR>(sm, stage ^ 1, (b + 1) & 1, min(FWD_BATCH, total - (b + 1) * FWD_BATCH),
+                                         K, geo, features, mask, depths);
+            cp_async_commit();
         }
         // (B) ids of batch b+2 into a register
         uint32_t next_id = 0;
@@ -254,12 +195,7 @@ render_forward_body(const uint2* __restrict__ ranges, const uint32_t* __restrict
 
         // (D) publish ids(b+2); wait for batch b+1
         if (have_next_id) sm.ids[b & 1][tid] = next_id;
-        if constexpr (TMA) {
-            // stage s is filled by batches b = s, s + 2, ...: its (b >> 1)-th fill completes phase parity (b >> 1) & 1
-            if (b + 1 < nbatch) mbarrier_wait_parity(&sm.bar[stage ^ 1], (uint32_t)(((b + 1) >> 1) & 1));
-        } else {
-            cp_async_wait_all();
-        }
+        cp_async_wait_all();
         if (b + 1 < nbatch) fwd_pad_batch<NQ>(sm, stage ^ 1, min(FWD_BATCH, total - (b + 1) * FWD_BATCH));
         __syncthreads();
     }
@@ -279,28 +215,5 @@ render_forward_body(const uint2* __restrict__ ranges, const uint32_t* __restrict
         }
     }
 }
-
-#define SAGARS_FWD_PARAMS                                                                                        \
-    const uint2* __restrict__ ranges, const uint32_t* __restrict__ point_list, int W, int H, int K,                 \
-    const float* __restrict__ geo, const float* __restrict__ features, const float* __restrict__ mask,              \
-    const float* __restrict__ depths, const float* __restrict__ bg, float* __restrict__ final_T,                    \
-    uint32_t* __restrict__ n_contrib, float* __restrict__ out_color, float* __restrict__ out_mask,                  \
-    float* __restrict__ out_depth
-#define SAGARS_FWD_ARGS ranges, point_list, W, H, K, geo, features, mask, depths, bg, final_T, n_contrib, out_color, out_mask, out_depth
-
-// cp.async (LDGSTS) staging -- the default
-template <int NQ, bool VEC, bool MD, bool COLOR>
-__global__ void __launch_bounds__(TILE_PIX) render_forward_kernel(SAGARS_FWD_PARAMS)
-{
-    render_forward_body<NQ, VEC, MD, COLOR, false>(SAGARS_FWD_ARGS);
-}
-// bulk-copy (TMA unit) staging completing on mbarriers -- SAGARS_FLAG_STAGE_TMA
-template <int NQ, bool VEC, bool MD, bool COLOR>
-__global__ void __launch_bounds__(TILE_PIX) render_forward_tma_kernel(SAGARS_FWD_PARAMS)
-{
-    render_forward_body<NQ, VEC, MD, COLOR, true>(SAGARS_FWD_ARGS);
-}
-#undef SAGARS_FWD_PARAMS
-#undef SAGARS_FWD_ARGS
 
 }  // namespace sagars

@@ -12,12 +12,6 @@
 
 namespace sagars {
 
-// SAGARS_FW_BULK = 1: the feature rows of a group (K == ROW: full 16-byte-multiple rows) are fetched by the TMA unit, one
-// cp.async.bulk per row completing on an mbarrier (8 copies from 8 lanes instead of 64 cp.async from 32); 0: cp.async pieces.
-#ifndef SAGARS_FW_BULK
-#define SAGARS_FW_BULK 0
-#endif
-
 
 constexpr int FW_WS = 40;    // row stride (words) of the W tile
 constexpr int FW_N = 8;      // candidates per group = k extent of one mma step
@@ -41,7 +35,6 @@ struct FwSmem {
     float4 ctab[FW_TAB][2];               // candidate records (x, y, cx, cy | cz, opacity, accept_threshold, -), list order
     uint32_t cid[FW_TAB];                 // their Gaussian ids
     float4 stage[2][32][2];               // the next chunk's records, one 32-byte slot per lane (cp.async, double buffered)
-    uint64_t fbar;                        // mbarrier of the feature-row bulk copies (SAGARS_FW_BULK)
 };
 
 // NQ : float4 groups covering the K colour channels;  VEC: K % 4 == 0 -> feature rows are read as float4
@@ -84,11 +77,6 @@ render_forward_warp_kernel(const uint2* __restrict__ ranges, const uint32_t* __r
     const uint32_t lt = (1u << lane) - 1u;
     float* const rowW = &sm.rowW[0][0];
     float* const Ft = &sm.F[0][0];
-    uint32_t fphase = 0;
-    if (SAGARS_FW_BULK) {
-        if (lane == 0) { mbarrier_init(&sm.fbar, 1); fence_proxy_async_smem(); }
-        __syncwarp();
-    }
 
     // one group: candidates in table slots [gs, gs + m), m <= 8
     auto process_group = [&](int gs, int m) {
@@ -107,7 +95,7 @@ render_forward_warp_kernel(const uint2* __restrict__ ranges, const uint32_t* __r
                 const uint32_t id = sm.cid[gs + min(r, m - 1)];
                 const int c0 = 4 * qd;
                 if (direct) {
-                    if (!SAGARS_FW_BULK) cp_async16(Ft + r * RS + 4 * qd, features + (size_t)id * K + c0);
+                    cp_async16(Ft + r * RS + 4 * qd, features + (size_t)id * K + c0);
                 } else if (VEC) {
                     if (c0 < K) fv[l] = __ldg(reinterpret_cast<const float4*>(features + (size_t)id * K + c0));
                 } else {
@@ -119,17 +107,7 @@ render_forward_warp_kernel(const uint2* __restrict__ ranges, const uint32_t* __r
                 }
             }
         }
-        if (direct) {
-            if (SAGARS_FW_BULK) {
-                // the MMA of the previous group has consumed the tile (its LDS results fed the HMMAs; __syncwarp at its end)
-                if (lane == 0) mbarrier_arrive_expect_tx(&sm.fbar, (uint32_t)(FW_N * ROW * sizeof(float)));
-                __syncwarp();
-                if (lane < FW_N)
-                    bulk_copy_g2s(Ft + lane * RS, features + (size_t)sm.cid[gs + min(lane, m - 1)] * K, (uint32_t)(ROW * sizeof(float)), &sm.fbar);
-            } else {
-                cp_async_commit();
-            }
-        }
+        if (direct) cp_async_commit();
         // The reference's chain as selects (no divergent branch, so the chains of neighbouring candidates interleave).  Tc is the
         // transmittance the chain tests with: it drops to 0 when the pixel saturates (or lies outside the image), after which
         // every test_T is 0 < 1e-4 and nothing is accepted -- no separate `done` flag; T keeps the value the reference reports.
@@ -163,8 +141,7 @@ render_forward_warp_kernel(const uint2* __restrict__ ranges, const uint32_t* __r
             }
         }
         if (direct) {
-            if (SAGARS_FW_BULK) { mbarrier_wait_parity(&sm.fbar, fphase); fphase ^= 1u; }
-            else cp_async_wait_all();
+            cp_async_wait_all();
         } else {
 #pragma unroll
             for (int l = 0; l < NLD; l++) {

@@ -139,8 +139,6 @@ def _flags(settings: GaussianRasterizationSettings, extra: int = 0) -> int:
         f |= _lib.FLAG_BWD_TILE
     elif _BACKWARD_KERNEL == "tc":
         f |= _lib.FLAG_BWD_TC
-    if _STAGING == "tma":
-        f |= _lib.FLAG_STAGE_TMA
     if _BINNING == "tile_sort":
         f |= _lib.FLAG_TILE_SORT
     elif _BINNING == "depth_first":
@@ -154,8 +152,6 @@ _FORWARD_KERNEL = "default"    # "default": mma.sync warp kernel at K = 32, fp32
                                # K = 32; "warp_any": the warp kernel for every colour-only channel count
 _BACKWARD_KERNEL = "default"   # "default": one warp per 8x4 pixel block (mma.sync); "tile": one CTA per 16x16 tile (mma.sync);
                                # "tc": tcgen05 / TMEM kernel, one CTA per 16x8 pixel group (C = 32 precomputed colours)
-_STAGING = "cp_async"          # how the tile-per-CTA fp32 forward gathers a batch into shared memory: "cp_async" (16-byte LDGSTS
-                               # pieces) or "tma" (one cp.async.bulk per row completing on an mbarrier; opt-in until measured)
 _BINNING = "depth_first"       # "depth_first" (default): Gaussians sorted by depth, instances emitted in that order, one stable sort on
                                # the tile bits; "radix": the reference's scheme -- global LSD radix sort of the duplicated tile|depth
                                # keys; "tile_sort": per-tile counts -> scan -> scatter -> one CTA per tile sorts its segment
@@ -188,15 +184,6 @@ def set_blend_kernels(forward: str = "default", backward: str = "default") -> No
     if forward not in ("default", "tile", "warp_any") or backward not in ("default", "tile", "tc"):
         raise ValueError("forward in {'default', 'tile', 'warp_any'}, backward in {'default', 'tile', 'tc'}")
     _FORWARD_KERNEL, _BACKWARD_KERNEL = forward, backward
-
-
-def set_staging(engine: str = "cp_async") -> None:
-    """Shared-memory staging engine of the tile-per-CTA fp32 forward (BASE / DEPTH / channel counts other than 32):
-    "cp_async" (default) or "tma" (bulk asynchronous copies on the TMA unit, ``SAGARS_FLAG_STAGE_TMA``).  Same results."""
-    global _STAGING
-    if engine not in ("cp_async", "tma"):
-        raise ValueError("engine in {'cp_async', 'tma'}")
-    _STAGING = engine
 
 
 _BLEND_WAIT_EVENT = None       # torch.cuda.Event the NEXT forward's blend stage waits for (set_blend_wait_event)

@@ -1,24 +1,13 @@
 // Host restatement of the entry points of seganygaussians_b200/csrc/cp_async.cuh for the CPU execution shim.
-// TEST INFRASTRUCTURE ONLY.  Asynchronous copies are made to land as LATE as the programming model allows:
-//   * cp.async pieces wait in a per-thread list until that thread's cp.async.wait_group / wait_all retires their group
-//     (or the thread leaves the kernel);
-//   * bulk copies wait on their mbarrier until some thread actually waits for that barrier's phase -- the waiting thread then
-//     plays the copy engine.  The mbarrier itself follows the PTX model: a phase completes when the pending arrival count
-//     AND the transaction count reach zero; complete_tx may run ahead of expect_tx (the count goes negative meanwhile).
-// A consumer that reads staged data before the matching wait therefore reads stale bytes, and a byte count or phase-parity
-// mistake ends in the 20-second timeout below instead of a silent pass.
-// -DSAGARS_EMU_ASYNC_EAGER flips to the other extreme: every copy lands the moment it is issued (the transaction count of a bulk
-// copy drops at once too).  A kernel that refills a buffer its threads are still reading -- a write-after-read hazard the "late"
-// mode cannot see -- then computes on the wrong data.  The suites run the staged kernels under both extremes.
+// TEST INFRASTRUCTURE ONLY.  Asynchronous copies are made to land as LATE as the programming model allows: cp.async pieces
+// wait in a per-thread list until that thread's cp.async.wait_group / wait_all retires their group (or the thread leaves the
+// kernel).  A consumer that reads staged data before the matching wait therefore reads stale bytes.
+// -DSAGARS_EMU_ASYNC_EAGER flips to the other extreme: every copy lands the moment it is issued.  A kernel that refills a buffer
+// its threads are still reading -- a write-after-read hazard the "late" mode cannot see -- then computes on the wrong data.  The
+// suites run the staged kernels under both extremes.
 #pragma once
-#include <chrono>
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <deque>
-#include <map>
-#include <mutex>
-#include <condition_variable>
 #include <vector>
 
 namespace sagars {
@@ -51,22 +40,6 @@ inline void flush_thread()
     retire(open_group);
 }
 
-struct Bulk { void* dst; const void* src; uint32_t bytes; };
-struct MBar {
-    int init = 0, pending = 0;
-    long long tx = 0;
-    unsigned phase = 0;                       // parity of the phase that is currently incomplete
-    std::vector<Bulk> in_flight;
-};
-inline std::mutex mu;
-inline std::condition_variable cv;
-inline std::map<const void*, MBar> bars;
-
-inline void check_complete(MBar& b)
-{
-    if (b.pending == 0 && b.tx == 0) { b.phase ^= 1u; b.pending = b.init; cv.notify_all(); }
-}
-
 }  // namespace emu_async
 
 #if defined(SAGARS_EMU_ASYNC_EAGER)
@@ -83,60 +56,6 @@ inline void cp_async_commit()
 }
 inline void cp_async_wait_all() { emu_async::flush_thread(); }
 template <int N> inline void cp_async_wait_group() { emu_async::retire_all_but((size_t)N); }
-
-inline void mbarrier_init(uint64_t* bar, uint32_t arrivals)
-{
-    std::lock_guard<std::mutex> lk(emu_async::mu);
-    emu_async::MBar& b = emu_async::bars[bar];
-    b = emu_async::MBar();
-    b.init = b.pending = (int)arrivals;
-}
-inline void fence_proxy_async_smem() {}
-inline void mbarrier_arrive_expect_tx(uint64_t* bar, uint32_t tx_bytes)
-{
-    std::lock_guard<std::mutex> lk(emu_async::mu);
-    emu_async::MBar& b = emu_async::bars.at(bar);
-    b.tx += tx_bytes;
-    b.pending -= 1;
-    if (b.pending < 0) { std::fprintf(stderr, "[cuda_emu] mbarrier: more arrivals than initialised\n"); std::abort(); }
-    emu_async::check_complete(b);
-}
-inline void bulk_copy_g2s(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar)
-{
-    if (bytes % 16u || ((uintptr_t)smem_dst & 15u) || ((uintptr_t)gmem_src & 15u)) {
-        std::fprintf(stderr, "[cuda_emu] cp.async.bulk: size / address not a multiple of 16 (%u bytes)\n", bytes);
-        std::abort();
-    }
-    std::lock_guard<std::mutex> lk(emu_async::mu);
-#if defined(SAGARS_EMU_ASYNC_EAGER)
-    emu_async::MBar& b = emu_async::bars.at(bar);
-    std::memcpy(smem_dst, gmem_src, bytes);
-    b.tx -= bytes;                                         // may run ahead of expect_tx, as the model allows
-    emu_async::check_complete(b);
-#else
-    emu_async::bars.at(bar).in_flight.push_back({smem_dst, gmem_src, bytes});
-#endif
-}
-inline void mbarrier_wait_parity(uint64_t* bar, uint32_t parity)
-{
-    std::unique_lock<std::mutex> lk(emu_async::mu);
-    emu_async::MBar& b = emu_async::bars.at(bar);
-    const auto deadline = std::chrono::steady_clock::now() + std::chrono::seconds(20);
-    for (;;) {
-        if (b.phase != (parity & 1u)) return;              // the phase with this parity has completed
-        if (!b.in_flight.empty()) {                        // play the copy engine: the data lands only now
-            std::vector<emu_async::Bulk> work;
-            work.swap(b.in_flight);
-            for (auto& c : work) { std::memcpy(c.dst, c.src, c.bytes); b.tx -= c.bytes; }
-            emu_async::check_complete(b);
-            continue;
-        }
-        if (emu_async::cv.wait_until(lk, deadline) == std::cv_status::timeout) {
-            std::fprintf(stderr, "[cuda_emu] mbarrier wait timed out: parity %u, pending %d, tx %lld\n", parity, b.pending, b.tx);
-            std::abort();
-        }
-    }
-}
 
 inline void red_add(float* addr, float a)
 {

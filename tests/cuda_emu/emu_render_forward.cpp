@@ -1,37 +1,11 @@
-// Host harness: the fp32 tile-per-CTA forward (seganygaussians_b200/csrc/render_forward_kernels.cuh) under the execution shim,
-// with either staging engine (cp.async pieces / bulk copies on mbarriers).  TEST INFRASTRUCTURE ONLY.
+// Host harness: the fp32 tile-per-CTA forward (seganygaussians_b200/csrc/render_forward_kernels.cuh) under the execution shim.
+// TEST INFRASTRUCTURE ONLY.
 #define SAGARS_CUDA_EMU 1
 #include <cuda_runtime.h>            // the shim (this directory comes first on the include path)
 #include "render_forward_kernels.cuh"
 #include "math.cuh"
 
 using namespace sagars;
-
-template <int NQ, bool VEC, bool MD>
-static void run(bool tma, int tiles_x, int tiles_y, const uint2* ranges, const uint32_t* point_list, int W, int H, int K,
-                const float* geo, const float* features, const float* mask, const float* depths, const float* bg,
-                float* final_T, uint32_t* n_contrib, float* out_color, float* out_mask, float* out_depth)
-{
-    cuda_emu::thread_exit_hook = emu_async::flush_thread;
-    const unsigned grid = (unsigned)(tiles_x * tiles_y);
-    // 1-D launch: the kernels read blockIdx.x / blockIdx.y and gridDim.x, so the harness walks the tiles row by row
-    for (int ty = 0; ty < tiles_y; ty++) {
-        struct RowLaunch {
-            static void go(bool tma_, int ty_, int tiles_x_, const uint2* r, const uint32_t* pl, int W_, int H_, int K_, const float* g,
-                           const float* f, const float* m, const float* d, const float* b, float* fT, uint32_t* nc, float* oc,
-                           float* om, float* od)
-            {
-                blockIdx.y = (unsigned)ty_;
-                if (tma_) render_forward_body<NQ, VEC, MD, true, true>(r, pl, W_, H_, K_, g, f, m, d, b, fT, nc, oc, om, od);
-                else render_forward_body<NQ, VEC, MD, true, false>(r, pl, W_, H_, K_, g, f, m, d, b, fT, nc, oc, om, od);
-            }
-        };
-        const size_t smem = sizeof(FwdSmemTma<NQ>) + 64;
-        cuda_emu::launch((unsigned)tiles_x, TILE_PIX, smem, RowLaunch::go, tma, ty, tiles_x, ranges, point_list, W, H, K, geo, features,
-                         mask, depths, bg, final_T, n_contrib, out_color, out_mask, out_depth);
-    }
-    (void)grid;
-}
 
 // the 32-byte records the preprocess kernel writes: {x, y, conic.x, conic.y, conic.z, opacity, accept_threshold, 0}
 extern "C" void emu_make_geo(int P, const float* means2D, const float* conic_opacity, float* geo)
@@ -44,14 +18,16 @@ extern "C" void emu_make_geo(int P, const float* means2D, const float* conic_opa
     }
 }
 
-extern "C" int emu_render_forward(int tma, int md, int W, int H, int K, const uint2* ranges, const uint32_t* point_list,
+extern "C" int emu_render_forward(int md, int W, int H, int K, const uint2* ranges, const uint32_t* point_list,
                                   const float* geo, const float* features, const float* mask, const float* depths, const float* bg,
                                   float* final_T, uint32_t* n_contrib, float* out_color, float* out_mask, float* out_depth)
 {
-    const int tx = (W + TILE_X - 1) / TILE_X, ty = (H + TILE_Y - 1) / TILE_Y;
+    cuda_emu::thread_exit_hook = emu_async::flush_thread;
+    const unsigned tx = (W + TILE_X - 1) / TILE_X, ty = (H + TILE_Y - 1) / TILE_Y;
     const bool vec = (K % 4) == 0;
     const int nq = (K + 3) / 4;
-#define GO(NQ_, VEC_, MD_) run<NQ_, VEC_, MD_>(tma != 0, tx, ty, ranges, point_list, W, H, K, geo, features, mask, depths, bg, final_T, n_contrib, out_color, out_mask, out_depth)
+#define GO(NQ_, VEC_, MD_) cuda_emu::launch2d(tx, ty, TILE_PIX, sizeof(FwdSmem<NQ_>), render_forward_kernel<NQ_, VEC_, MD_, true>, ranges, point_list, \
+                                              W, H, K, geo, features, mask, depths, bg, final_T, n_contrib, out_color, out_mask, out_depth)
     if (md) { if (nq == 1 && !vec) { GO(1, false, true); return 0; } return -1; }
     if (nq == 1 && !vec) { GO(1, false, false); return 0; }
     if (nq == 2 && vec) { GO(2, true, false); return 0; }

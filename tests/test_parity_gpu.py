@@ -342,30 +342,6 @@ def test_blend_kernel_variants_agree(cfg):
         assert ok, (key, report)
 
 
-
-@pytest.mark.parametrize("cfg", [("base", 4000, 90, 130, 3, False), ("depth", 4000, 90, 130, 3, True), ("k16", 2500, 80, 96, 16, False),
-                                 ("k32", 3000, 72, 104, 32, False), ("k64", 1500, 64, 80, 64, False), ("k5", 1500, 64, 80, 5, False),
-                                 ("long_lists", 6000, 48, 48, 8, False)],
-                         ids=lambda c: c[0])
-def test_tma_staging_is_bit_identical(cfg):
-    """SAGARS_FLAG_STAGE_TMA only changes HOW a batch reaches shared memory (cp.async.bulk rows on mbarriers instead of
-    16-byte cp.async pieces): every output of the fp32 tile forward must be bit-identical."""
-    from seganygaussians_b200 import rasterizer as R
-    name, P, H, W, K, depth = cfg
-    sc = synthetic.scene(P, H, W, K, sigma_px=6.0 if name == "long_lists" else 2.0)
-    try:
-        R.set_staging("cp_async")
-        a = common.run_torch_impl("ours", sc, K, depth=depth, tensor_cores=False, backward=False)
-        R.set_staging("tma")
-        b = common.run_torch_impl("ours", sc, K, depth=depth, tensor_cores=False, backward=False)
-    finally:
-        R.set_staging("cp_async")
-    for f in ("color", "final_T", "n_contrib", "out_mask", "out_depth"):
-        x, y = getattr(a, f), getattr(b, f)
-        if x is not None:
-            assert np.array_equal(x, y), f
-
-
 @pytest.mark.parametrize("mod", [0.6, 1.7])
 def test_scale_modifier_matches_oracle(mod):
     """scale_modifier != 1 (the viewer's scaling slider): forward state and every gradient against the CPU oracle, including the

@@ -1,11 +1,7 @@
 """The fp32 tile-per-CTA forward kernel (seganygaussians_b200/csrc/render_forward_kernels.cuh) executed on the CPU under the
-CUDA execution shim, with BOTH staging engines:
-
-  * cp.async pieces (the default, GPU-validated) -- keeps the product kernel's control flow (double-buffered batches, sentinel
-    padding, early exit, ragged edges) under test in the CPU-only suite;
-  * bulk copies on mbarriers (SAGARS_FLAG_STAGE_TMA, not yet run on a GPU) -- the shim models the mbarrier of the PTX ISA
-    (pending arrivals + transaction bytes, phase parity) and lets every asynchronous copy land as LATE as the model allows, so
-    a wrong byte count, a wrong phase parity or a read before the wait fails here (time-out / stale data) instead of on the GPU.
+CUDA execution shim.  Keeps the kernel's control flow (cp.async staging of double-buffered batches, sentinel padding, early
+exit, ragged edges) under test in the CPU-only suite; the shim lets every asynchronous copy land as late, or as early, as the
+programming model allows, so a read before the wait or a buffer refilled while still in use computes on the wrong data.
 
 Compared with the CPU oracle: n_contrib exact, final_T / colours / mask / depth to fp32 rounding (the host compiler does not
 contract a*b+c the way nvcc does, so the last bit of `power` may differ; 5e-6 relative is ample)."""
@@ -35,12 +31,12 @@ def emu(request):
                            os.path.join(ROOT, "tests", "cuda_emu", "emu_render_forward.cpp"), "-o", so])
     L = C.CDLL(so)
     L.emu_render_forward.restype = C.c_int
-    L.emu_render_forward.argtypes = [C.c_int] * 5 + [C.c_void_p] * 12
+    L.emu_render_forward.argtypes = [C.c_int] * 4 + [C.c_void_p] * 12
     L.emu_make_geo.argtypes = [C.c_int] + [C.c_void_p] * 3
     return L
 
 
-def _render(emu, o, sc, K, tma, depth, bg):
+def _render(emu, o, sc, K, depth, bg):
     P, H, W = sc.P, sc.H, sc.W
     geo = np.zeros((P, 8), np.float32)
     m2 = np.ascontiguousarray(o.means2D.astype(np.float32))
@@ -58,7 +54,7 @@ def _render(emu, o, sc, K, tma, depth, bg):
     out = dict(final_T=np.zeros((H, W), np.float32), n_contrib=np.zeros((H, W), np.uint32), color=np.zeros((K, H, W), np.float32),
                out_mask=np.zeros((1, H, W), np.float32), out_depth=np.zeros((1, H, W), np.float32))
     bg = np.ascontiguousarray(bg.astype(np.float32))
-    rc = emu.emu_render_forward(int(tma), int(depth), W, H, K, p(ranges), p(pl), p(geo), p(feats), p(mask), p(depths), p(bg),
+    rc = emu.emu_render_forward(int(depth), W, H, K, p(ranges), p(pl), p(geo), p(feats), p(mask), p(depths), p(bg),
                                 p(out["final_T"]), p(out["n_contrib"]), p(out["color"]), p(out["out_mask"]), p(out["out_depth"]))
     assert rc == 0
     return out
@@ -74,9 +70,8 @@ CASES = [
 ]
 
 
-@pytest.mark.parametrize("tma", [False, True], ids=["cp_async", "tma"])
 @pytest.mark.parametrize("case", CASES, ids=[c[0] for c in CASES])
-def test_emulated_forward_matches_oracle(emu, case, tma):
+def test_emulated_forward_matches_oracle(emu, case):
     name, P, H, W, K, depth, sigma = case
     sc = synthetic.scene(P, H, W, K, sigma_px=sigma)
     import torch
@@ -84,7 +79,7 @@ def test_emulated_forward_matches_oracle(emu, case, tma):
     o = common.run_oracle(sc, K, depth=depth, backward=False, bg=torch.tensor(bg))
     if name != "short_lists":
         assert (o.ranges[:, 1].astype(np.int64) - o.ranges[:, 0]).max() > 130     # at least three batches somewhere
-    out = _render(emu, o, sc, K, tma, depth, bg)
+    out = _render(emu, o, sc, K, depth, bg)
     assert np.array_equal(out["n_contrib"], o.n_contrib)
     np.testing.assert_allclose(out["final_T"], o.final_T, rtol=5e-6, atol=1e-9)
     np.testing.assert_allclose(out["color"], o.color, rtol=5e-6, atol=2e-7)

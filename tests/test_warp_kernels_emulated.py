@@ -34,17 +34,6 @@ def _build_emu(extra):
     return so
 
 
-@pytest.fixture(scope="module", params=["late", "eager"])
-def emu_bulk(request):
-    """The forward warp kernel with its feature rows fetched by bulk copies on an mbarrier (-DSAGARS_FW_BULK=1: the TMA-unit variant
-    measured against the cp.async default in round 2, profiles/r2_render_kernels.md)."""
-    L = C.CDLL(_build_emu(["-DSAGARS_FW_BULK=1"] + (["-DSAGARS_EMU_ASYNC_EAGER"] if request.param == "eager" else [])))
-    L.emu_forward_warp.restype = C.c_int
-    L.emu_forward_warp.argtypes = [C.c_int] * 3 + [C.c_void_p] * 8
-    L.emu_make_geo.argtypes = [C.c_int] + [C.c_void_p] * 3
-    return L
-
-
 # "eager": asynchronous copies land the moment they are issued (the other extreme of what the programming model allows): a buffer
 # refilled while it is still being read shows up as wrong results
 @pytest.fixture(scope="module", params=["default", "eager"])
@@ -98,16 +87,6 @@ def _inputs(emu, fw, sc, K):
                                   ("k5", 260, 32, 32, 5, 5.0),
                                   ("k3_warp_any", 300, 32, 32, 3, 5.0)], ids=lambda c: c[0])
 def test_forward_warp_kernel(emu, case):
-    _forward_warp_case(emu, case)
-
-
-@pytest.mark.parametrize("case", [("k32", 260, 32, 32, 32, 5.0), ("k32_ragged", 200, 27, 41, 32, 4.0), ("k32_opaque", 260, 32, 32, 32, 5.0)],
-                         ids=lambda c: c[0])
-def test_forward_warp_kernel_bulk_copy_variant(emu_bulk, case):
-    _forward_warp_case(emu_bulk, case)
-
-
-def _forward_warp_case(emu, case):
     name, P, H, W, K, sigma = case
     sc = synthetic.scene(P, H, W, K, sigma_px=sigma)
     if name == "k32_opaque":

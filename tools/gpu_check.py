@@ -96,15 +96,15 @@ def sort_check():
     return ok_all
 
 
-def timing(P, H, W, K, iters=10, depth=False, use_sh=False, deg=0, M=0, only_ours=False, tag=""):
-    section(f"timing{tag}: P={P} {H}x{W} K={K} depth={depth} sh={use_sh}")
+def timing(P, H, W, K, iters=10, depth=False, use_sh=False, deg=0, M=0):
+    section(f"timing: P={P} {H}x{W} K={K} depth={depth} sh={use_sh}")
     dev = torch.device("cuda", 0)
     sc = synthetic.scene(P, H, W, K, sh_coeffs=M)
     variant = common.variant_of(K, depth)
     from seganygaussians_b200 import rasterizer as R
     impls = {"ours": (R.GaussianRasterizationSettings, {"base": R.GaussianRasterizer, "cf": R.GaussianRasterizerContrastiveF,
                                                         "depth": R.GaussianRasterizerDepth}[variant])}
-    if common.have_ref(variant) and not only_ours:
+    if common.have_ref(variant):
         m = common.ref_module(variant)
         impls["ref"] = (m.GaussianRasterizationSettings, m.GaussianRasterizer)
     g = sc.gauss
@@ -144,8 +144,6 @@ if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("--tiny", action="store_true", help="only the smallest parity case (for compute-sanitizer)")
     ap.add_argument("--no-timing", action="store_true")
-    ap.add_argument("--staging-ab", action="store_true",
-                    help="time the tile-per-CTA fp32 forward with cp.async staging vs bulk-copy (TMA unit) staging (SAGARS_FLAG_STAGE_TMA)")
     ap.add_argument("--large", action="store_true", help="BASELINE-scale parity + timing of the other configs (c1, c3-like, c5-like)")
     a = ap.parse_args()
     print("device:", torch.cuda.get_device_name(0), "| lib:", _lib.load().sagars_arch().decode())
@@ -155,17 +153,6 @@ if __name__ == "__main__":
         results["tiny_depth"] = parity("tiny_depth", 500, 40, 56, 3, depth=True, with_ref=False)
         print(results)
         sys.exit(0 if all(results.values()) else 1)
-    if a.staging_ab:
-        from seganygaussians_b200 import rasterizer as R
-        R.set_tensor_cores(False)   # K = 32 through the fp32 tile kernel too
-        for eng in ("cp_async", "tma"):
-            R.set_staging(eng)
-            timing(1000000, 1080, 1920, 3, iters=10, only_ours=True, tag=f" [{eng}]")
-            timing(2000000, 1600, 1600, 3, iters=5, depth=True, use_sh=True, deg=3, M=16, only_ours=True, tag=f" [{eng}]")
-            timing(1000000, 1080, 1920, 16, iters=10, only_ours=True, tag=f" [{eng}]")
-            timing(1000000, 1080, 1920, 32, iters=10, only_ours=True, tag=f" [{eng}]")
-        R.set_staging("cp_async")
-        sys.exit(0)
     if a.large:
         results["c1"] = parity("c1", 10000, 256, 256, 3, with_oracle=True)
         results["c3_like"] = parity("c3_like", 5000000, 1036, 1600, 32, with_oracle=False)

@@ -1,10 +1,10 @@
 #!/usr/bin/env bash
 # compute-sanitizer over the small parity tests (SURVEY.md section 5, "race detection / sanitizers"): every blend-kernel variant,
-# the three binning methods, the bulk-copy staging, the fused smoothing / sampling ops and the KNN.  memcheck = out-of-bounds /
+# the three binning methods, the fused smoothing / sampling ops and the KNN.  memcheck = out-of-bounds /
 # misaligned accesses; racecheck = shared-memory hazards; synccheck = divergent barriers.  One GPU.
 set -u
 mkdir -p gpurun_out
-SEL='test_blend_kernel_variants_agree or test_depth_first_binning_is_bit_identical or test_tile_sort_binning_is_bit_identical or test_tma_staging_is_bit_identical or test_edge_cases or test_mask_only_path or test_cuda_matches_oracle'
+SEL='test_blend_kernel_variants_agree or test_depth_first_binning_is_bit_identical or test_tile_sort_binning_is_bit_identical or test_edge_cases or test_mask_only_path or test_cuda_matches_oracle'
 for tool in memcheck racecheck synccheck; do
   echo "== compute-sanitizer --tool $tool =="
   timeout 200 compute-sanitizer --tool $tool --error-exitcode 77 --log-file gpurun_out/r2_sanitizer_${tool}.log \
